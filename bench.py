@@ -24,6 +24,8 @@ import sys
 import tempfile
 import time
 
+sys.dont_write_bytecode = True  # the tree may be read-only: no __pycache__ next to the sources
+
 # the prover uses more streams than the driver's default 8 hardware queues (see csrc/cs_api.cu); must be set before the
 # CUDA context exists
 os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")
@@ -428,7 +430,7 @@ def run_ours(args):
         e0.record(stream)
         tw0 = time.perf_counter()
         for _ in range(args.steps):
-            pk.prove_plain_device(pub, d_wit, r_m, s_m)
+            proof = pk.prove_plain_device(pub, d_wit, r_m, s_m)
         e1.record(stream)
     torch.cuda.synchronize()
     tw1 = time.perf_counter()
@@ -437,6 +439,8 @@ def run_ours(args):
     value_ms = max_over_ranks(max(dev_ms, (tw1 - tw0) * 1e3))
     launches = ctx.launch_count() - l0
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(("proof_a", "proof_b", "proof_c"), proof)))
 
     timeline = None
     if args.timeline and rank == 0:
@@ -597,6 +601,16 @@ def run_ours(args):
         print(json.dumps(out))
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes each uint64 limb array as out_dir/<name>.npy: its 32-bit words (little-endian order) as float64, which
+    holds them exactly, so two builds can be compared word for word."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        words = np.ascontiguousarray(a, dtype=np.uint64).view(np.uint32).astype(np.float64)
+        np.save(os.path.join(out_dir, name + ".npy"), words)
+
+
 def ncu_traffic():
     """dram__bytes_read.sum + dram__bytes_write.sum of the accumulate kernel from the committed ncu summary."""
     path = os.path.join(ROOT, "profiles", "r2_ncu_full_accum0_g1.csv")
@@ -736,7 +750,12 @@ def main():
     ap.add_argument("--timeline", action="store_true",
                     help="after the timed region: one more proof with stage events, reported as timeline_ms (diagnostic)")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="diagnostic runs: skip the CPU leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the proof (A, B, C) of the last timed step as DIR/proof_{a,b,c}.npy: the affine Montgomery "
+                         "limbs the prover returns, as float64 32-bit words")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

@@ -56,6 +56,40 @@ def dump(name, obj, compress=False):
     print(path, os.path.getsize(path))
 
 
+def compact_plonk_key(obj, p_tau_from=None):
+    """Shrinks a large Plonk key to what helpers.load_golden rebuilds it from: the selectors' evaluations over the
+    domain, the permutation as indices (i -> w^i, n + i -> k1 w^i, 2n + i -> k2 w^i), no Lagrange polynomials, and
+    optionally the p_tau points by reference to another fixture that holds the same ones."""
+    from oracle.fields import CURVES
+    r, n = CURVES[obj["curve"]].r, obj["domain_size"]
+    _, roots = roots_of_unity(r)
+    w = [1]
+    for _ in range(n - 1):
+        w.append(w[-1] * roots[n.bit_length() - 1] % r)
+    index = {hx(k * x % r): j * n + i for j, k in enumerate((1, int(obj["k1"], 16), int(obj["k2"], 16))) for i, x in enumerate(w)}
+    obj["q_domain_evals"] = {k: obj.pop(k)["evals"][0::4] for k in ("qm", "ql", "qr", "qo", "qc")}
+    obj["sigma"] = [[index[x] for x in obj.pop(k)["evals"][0::4]] for k in ("s1", "s2", "s3")]
+    del obj["lagrange"]
+    if p_tau_from:
+        assert load(p_tau_from)["p_tau"] == obj.pop("p_tau")
+        obj["p_tau_from"] = p_tau_from
+    return obj
+
+
+def compact_round1(obj, blinders):
+    """Drops each wire's polynomial and blinded polynomial: helpers.load_golden recomputes them from the wire values
+    and the blinders (the same steps as plonk_fixture)."""
+    for wire, blind in zip(obj["wires"], blinders):
+        del wire["poly"], wire["blinded"]
+        wire["blinders"] = blind
+    return obj
+
+
+def load(name):
+    p = os.path.join(HERE, name + ".json")
+    return json.load(gzip.open(p + ".gz") if not os.path.exists(p) else open(p))
+
+
 def groth16_fixture(name, r_s_list, compress, curve_dir="bn254"):
     groth16_verify = groth16_verify_bn254
     if curve_dir == "bls12_381":
@@ -121,7 +155,8 @@ def plonk_fixture(curve_dir, name, expected, compress):
     for s1, s2, f1, f2 in z["additions"]:
         additions.append((get_witness(s1) * f1 + get_witness(s2) * f2) % r)
     wires = []
-    for wire_map, blind in ((z["map_a"], [0, 1]), (z["map_b"], [2, 3]), (z["map_c"], [4, 5])):
+    blinders = [[0, 1], [2, 3], [4, 5]]
+    for wire_map, blind in zip((z["map_a"], z["map_b"], z["map_c"]), blinders):
         buf = [get_witness(i) for i in wire_map] + [0] * (n - len(wire_map))
         poly = ifft(buf, gen, r)
         rev = list(reversed(blind))
@@ -135,7 +170,7 @@ def plonk_fixture(curve_dir, name, expected, compress):
                expected_commitments=[p1(P) for P in expected],
                expected_source="co-circom/co-plonk/src/round1.rs:351-371" if curve_dir == "bn254" else
                "co-circom/co-plonk/src/round1.rs:397-417")
-    dump("plonk_round1_%s_%s" % (curve_dir, name), obj, compress)
+    dump("plonk_round1_%s_%s" % (curve_dir, name), compact_round1(obj, blinders) if compress else obj, compress)
 
 
 # The reference's known answers for the whole prover with deterministic blinders b[i] = i on BN254 multiplier2
@@ -171,7 +206,7 @@ VERIFIER_KAT = dict(  # plonk.rs:266-309, on the snarkjs proof of the same circu
     u=13260637895132000183831258130762201406791497612259050836989270998713858775580)
 
 
-def plonk_full_fixture(name, compress, curve_dir="bn254"):
+def plonk_full_fixture(name, compress, curve_dir="bn254", p_tau_from=None):
     """Everything the Plonk prover reads from the zkey (taceo-circom-types plonk::Zkey) + witness, verification
     key, public inputs, the snarkjs proof, and the reference's round 2-5 / verifier known answers."""
     from oracle import plonk as OP
@@ -215,6 +250,8 @@ def plonk_full_fixture(name, compress, curve_dir="bn254"):
         obj["reference_verifier_kat"] = dict(source="co-circom/co-plonk/src/plonk.rs:266-309",
                                              **{k: ([hx(x) for x in v] if isinstance(v, list) else hx(v))
                                                 for k, v in VERIFIER_KAT.items()})
+    if compress:
+        obj = compact_plonk_key(obj, p_tau_from)
     dump("plonk_full_%s_%s" % (curve_dir, name), obj, compress)
 
 
@@ -222,6 +259,30 @@ def crs_fixture(n):
     pts = F.read_bn254_crs_g1("%s/co-noir/co-noir-common/src/crs/bn254_g1.dat" % REF, n)
     dump("crs_bn254_g1_first%d" % n, dict(source="co-noir/co-noir-common/src/crs/bn254_g1.dat",
                                           points=[p1(P) for P in pts]), True)
+
+
+def reference_files():
+    """The reference's own files that the readers / ingest paths are tested on, under snarkjs/ (zkeys gzipped), and the
+    first 64 points of the Ignition CRS file, byte for byte."""
+    for rel in ("Groth16/bn254/multiplier2/circuit.zkey", "Groth16/bn254/multiplier2/witness.wtns",
+                "Groth16/bn254/poseidon/circuit.zkey", "Groth16/bn254/poseidon/witness.wtns",
+                "Groth16/bn254/poseidon/verification_key.json",
+                "Groth16/bls12_381/poseidon/circuit.zkey", "Groth16/bls12_381/poseidon/witness.wtns",
+                "Groth16/bls12_381/poseidon/verification_key.json", "Groth16/bls12_381/poseidon/circom.proof",
+                "Groth16/bls12_381/poseidon/public.json",
+                "Plonk/bn254/multiplier2/circuit.zkey", "Plonk/bls12_381/multiplier2/circuit.zkey",
+                "Plonk/bls12_381/poseidon/verification_key.json", "Plonk/bls12_381/poseidon/circom.proof",
+                "Plonk/bls12_381/poseidon/public.json"):
+        data = open("%s/test_vectors/%s" % (REF, rel), "rb").read()
+        dst = os.path.join(HERE, "snarkjs", rel)
+        os.makedirs(os.path.dirname(dst), exist_ok=True)
+        if rel.endswith(".zkey"):
+            with gzip.GzipFile(dst + ".gz", "wb", mtime=0) as f:
+                f.write(data)
+        else:
+            open(dst, "wb").write(data)
+    crs = open("%s/co-noir/co-noir-common/src/crs/bn254_g1.dat" % REF, "rb").read(64 * 64)
+    open(os.path.join(HERE, "crs_bn254_g1_first64.dat"), "wb").write(crs)
 
 
 if __name__ == "__main__":
@@ -245,4 +306,6 @@ if __name__ == "__main__":
     plonk_full_fixture("multiplier2", False)
     plonk_full_fixture("poseidon", True)
     plonk_full_fixture("multiplier2", False, "bls12_381")
+    plonk_full_fixture("poseidon", True, "bls12_381", p_tau_from="plonk_round1_bls12_381_poseidon")
     groth16_fixture("multiplier2", [(0, 0), (11, 13)], False, "bls12_381")
+    reference_files()

@@ -6,7 +6,8 @@ import os
 import numpy as np
 
 from co_snarks_b200 import binding as B
-from oracle.fields import CURVES
+from oracle.fields import CURVES, roots_of_unity
+from oracle.ntt import fft, ifft
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -16,7 +17,61 @@ def load_golden(name):
     if os.path.exists(p):
         return json.load(open(p))
     with gzip.open(p + ".gz", "rb") as f:
-        return json.loads(f.read().decode())
+        g = json.loads(f.read().decode())
+    if "sigma" in g:
+        _expand_plonk_key(g)
+    if "wires" in g and "blinders" in g["wires"][0]:
+        _expand_round1(g)
+    return g
+
+
+def _hx(v):
+    return format(v, "x")
+
+
+def _expand_plonk_key(g):
+    """Inverse of make_golden.compact_plonk_key: the polynomials in the zkey's layout (n coefficients, then the
+    evaluations over the 4n-point domain) from their evaluations over the n-point domain."""
+    r, n = CURVES[g["curve"]].r, g["domain_size"]
+    _, roots = roots_of_unity(r)
+    gen_n, gen_4n = roots[n.bit_length() - 1], roots[n.bit_length() + 1]
+
+    def poly(evals):
+        co = ifft(evals, gen_n, r)
+        return dict(coeffs=[_hx(x) for x in co], evals=[_hx(x) for x in fft(co + [0] * (3 * n), gen_4n, r)])
+    w = [1]
+    for _ in range(n - 1):
+        w.append(w[-1] * gen_n % r)
+    k = (1, ih(g["k1"]), ih(g["k2"]))
+    for name, ev in g.pop("q_domain_evals").items():
+        g[name] = poly([ih(x) for x in ev])
+    for name, sig in zip(("s1", "s2", "s3"), g.pop("sigma")):
+        g[name] = poly([k[s // n] * w[s % n] % r for s in sig])
+    g["lagrange"] = [poly([int(i == j) for i in range(n)]) for j in range(max(1, g["n_public"]))]
+    if "p_tau_from" in g:
+        g["p_tau"] = load_golden(g.pop("p_tau_from"))["p_tau"]
+
+
+def _expand_round1(g):
+    """Inverse of make_golden.compact_round1: each wire's polynomial and blinded polynomial."""
+    r = CURVES[g["curve"]].r
+    for wire in g["wires"]:
+        poly = ifft([ih(x) for x in wire["buffer"]], ih(g["group_gen"]), r)
+        rev = list(reversed(wire.pop("blinders")))
+        blinded = [(c - rev[i]) % r if i < len(rev) else c for i, c in enumerate(poly)] + rev
+        wire["poly"], wire["blinded"] = [_hx(x) for x in poly], [_hx(x) for x in blinded]
+
+
+def golden_fixture(tmp_dir, rel):
+    """Path of one of the reference's snarkjs test-vector files kept under golden/snarkjs/<rel>; a file stored
+    gzipped is unpacked into tmp_dir first, since the readers under test take a path."""
+    p = os.path.join(GOLDEN, "snarkjs", rel)
+    if os.path.exists(p):
+        return p
+    out = os.path.join(str(tmp_dir), rel.replace("/", "_"))
+    with gzip.open(p + ".gz", "rb") as f, open(out, "wb") as g:
+        g.write(f.read())
+    return out
 
 
 def ih(x):

@@ -9,7 +9,7 @@ import pytest
 import numpy as np
 
 from co_snarks_b200 import binding as B
-from helpers import Conv, golden_groth16, gp1, ih, load_golden, make_key
+from helpers import GOLDEN, Conv, golden_groth16, gp1, ih, load_golden, make_key
 from oracle import groth16 as OG
 from oracle import ntt as ON
 from oracle.ec import g1 as og1, g2 as og2
@@ -199,12 +199,11 @@ def check_crs_file_ingest(ctx, tmp_path):
         bases.free()
     with pytest.raises(RuntimeError):
         ctx.bases_from_crs_file(path, 400)  # more points than the file holds
-    ref = "/root/reference/co-noir/co-noir-common/src/crs/bn254_g1.dat"
-    if os.path.exists(ref):  # the real file, when mounted: first point is the generator
-        bases = ctx.bases_from_crs_file(ref, 64)
-        out, _ = ctx.msm(bases, cv.fr([1] + [0] * 63))
-        assert cv.pt1(out) == (1, 2)
-        bases.free()
+    # the first 64 points of the real file, byte for byte: its first point is the generator
+    bases = ctx.bases_from_crs_file(os.path.join(GOLDEN, "crs_bn254_g1_first64.dat"), 64)
+    out, _ = ctx.msm(bases, cv.fr([1] + [0] * 63))
+    assert cv.pt1(out) == (1, 2)
+    bases.free()
 
 
 def check_fixed_base_mul(ctx, n=40):
@@ -564,10 +563,10 @@ def check_plonk_prove(ctx, name="multiplier2", random_blinders=True, curve="bn25
 
 
 def check_plonk_zkey_ingest(ctx, tmp_path, name="multiplier2", curve="bn254"):
-    """cs_plonk_pk_from_zkey: a snarkjs-format Plonk .zkey written from the golden fixture (and the reference's own
-    file when /root/reference is mounted) goes straight to the device layout; the proof equals the golden one."""
+    """cs_plonk_pk_from_zkey: a snarkjs-format Plonk .zkey written from the golden fixture, and the reference's own
+    file, go straight to the device layout; the proof equals the golden one."""
     import os
-    from helpers import golden_plonk, plonk_proof_from_device
+    from helpers import golden_fixture, golden_plonk, plonk_proof_from_device
     from oracle import formats as F
     from zkey_writer import write_plonk_zkey
     cv = Conv(curve)
@@ -576,10 +575,7 @@ def check_plonk_zkey_ingest(ctx, tmp_path, name="multiplier2", curve="bn254"):
     write_plonk_zkey(path, z)
     back = F.read_plonk_zkey(path)
     assert all(back[k] == z[k] for k in ("k1", "k2", "map_a", "additions", "qm", "s3", "lagrange", "p_tau", "x2", "vk_s2"))
-    paths = [path]
-    ref = "/root/reference/test_vectors/Plonk/%s/%s/circuit.zkey" % (curve, name)
-    if os.path.exists(ref):
-        paths.append(ref)
+    paths = [path, golden_fixture(tmp_path, "Plonk/%s/%s/circuit.zkey" % (curve, name))]
     npub = z["n_public"]
     for pth in paths:
         pk = B.PlonkKey.from_zkey(ctx, pth, cv.id)
@@ -802,9 +798,10 @@ def check_shamir_degree_reduce(ctx, n=64, seed=12):
 def check_zkey_ingest(ctx, tmp_path, name="multiplier2"):
     """cs_groth16_pk_from_zkey + cs_wtns_read (co-circom.rs:1005-1016): a snarkjs-format key/witness pair goes
     file -> device and proves to the golden proof bytes; the writer's output is also parsed by the oracle's
-    reader, and -- when the reference tree is mounted -- the reference's own files are ingested too."""
+    reader, and the reference's own files are ingested too."""
     import os
     import zkey_writer
+    from helpers import golden_fixture
     from oracle import formats as OF
     from oracle.formats import proof_to_json
     cv = Conv("bn254")
@@ -814,10 +811,8 @@ def check_zkey_ingest(ctx, tmp_path, name="multiplier2"):
     zkey_writer.write_wtns(wp, cv.r, w)
     z2 = OF.read_groth16_zkey(zp)  # the test writer agrees with the oracle's reader
     assert z2["a_query"] == z["a_query"] and OF.zkey_matrices(z2)["a"] == m["a"]
-    files = [(zp, wp)]
-    ref = "/root/reference/test_vectors/Groth16/bn254/%s/" % name
-    if os.path.isdir(ref):
-        files.append((ref + "circuit.zkey", ref + "witness.wtns"))
+    ref = "Groth16/bn254/%s/" % name
+    files = [(zp, wp), (golden_fixture(tmp_path, ref + "circuit.zkey"), golden_fixture(tmp_path, ref + "witness.wtns"))]
     for zf, wf in files:
         pk = B.Groth16Key.from_zkey(ctx, zf)
         assert pk.domain_size() == g["domain_size"] and pk.ni == m["num_instance_variables"]

@@ -1,22 +1,20 @@
 """CPU-only: the Python oracle against the committed golden vectors (tests/golden/make_golden.py):
 the reference's Plonk round-1 known answers, the snarkjs proofs/verification keys of the reference's
-Groth16 fixtures, and -- when /root/reference is mounted -- the raw fixture files themselves."""
+Groth16 fixtures, and the raw fixture files themselves (tests/golden/snarkjs)."""
 import json
 import os
 import random
 
 import pytest
 
-from helpers import golden_groth16, golden_plonk, gp1, gp2, ih, load_golden, plonk_proof_from_json, plonk_vk_from_zkey
+from helpers import (GOLDEN, golden_fixture, golden_groth16, golden_plonk, gp1, gp2, ih, load_golden, plonk_proof_from_json,
+                     plonk_vk_from_zkey)
 from oracle import formats as F
 from oracle import groth16 as OG
 from oracle.ec import g1 as og1
 from oracle.fields import BLS12_381, BN254, CURVES, roots_of_unity
 from oracle.ntt import ifft
 from oracle.pairing_bn254 import groth16_verify
-
-REF = "/root/reference"
-
 
 @pytest.mark.parametrize("name", ["multiplier2", "poseidon"])
 def test_snarkjs_proof_verifies_and_oracle_proof_matches_golden(name):
@@ -60,19 +58,19 @@ def test_plonk_round1_kat(curve, name):
         assert G.msm(p_tau[:len(blinded)], blinded) == gp1(exp)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted (GPU box)")
-def test_file_parsers_agree_with_golden():
-    base = REF + "/test_vectors/Groth16/bn254/poseidon/"
-    z = F.read_groth16_zkey(base + "circuit.zkey")
+def test_file_parsers_agree_with_golden(tmp_path):
+    """The oracle's readers on the reference's own files (zkey, wtns, verification key, Ignition CRS)."""
+    base = "Groth16/bn254/poseidon/"
+    z = F.read_groth16_zkey(golden_fixture(tmp_path, base + "circuit.zkey"))
     m = F.zkey_matrices(z)
-    _, w = F.read_wtns(base + "witness.wtns")
+    _, w = F.read_wtns(golden_fixture(tmp_path, base + "witness.wtns"))
     zg, mg, wg, g = golden_groth16("poseidon")
     assert w == wg and m["a"] == mg["a"] and m["b"] == mg["b"]
     for k in ("a_query", "b_g2_query", "h_query", "l_query", "alpha_g1", "delta_g2"):
         assert z[k] == zg[k]
-    vk = F.read_vk_json(base + "verification_key.json")
+    vk = F.read_vk_json(golden_fixture(tmp_path, base + "verification_key.json"))
     assert vk["ic"] == z["ic"] and vk["gamma_g2"] == z["gamma_g2"]
-    pts = F.read_bn254_crs_g1(REF + "/co-noir/co-noir-common/src/crs/bn254_g1.dat", 4)
+    pts = F.read_bn254_crs_g1(os.path.join(GOLDEN, "crs_bn254_g1_first64.dat"), 4)
     assert pts[0] == (1, 2) and all(og1(BN254).on_curve(P) for P in pts)
 
 
@@ -162,43 +160,46 @@ def test_bls12_381_fixtures_verify():
     assert not OP.verify(BLS12_381, vkp, bad, pubp, ppio)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted (GPU box)")
-def test_bls12_381_poseidon_fixtures_from_the_reference_tree():
+def test_bls12_381_poseidon_fixtures_from_the_reference_tree(tmp_path):
     """co-groth16/src/lib.rs:122-160 (poseidon on BLS12-381): the snarkjs proof verifies; the oracle's proof from the
     fixture's zkey + witness verifies too.  Plonk: the snarkjs proof verifies (co-plonk/src/plonk.rs:332-350)."""
     from oracle import plonk as OP
     from oracle.fields import BLS12_381
     from oracle.pairing_bls12_381 import groth16_verify as verify_bls, pairing_product_is_one as ppio
-    base = REF + "/test_vectors/Groth16/bls12_381/poseidon/"
-    vk = F.read_vk_json(base + "verification_key.json")
-    public = [int(x) for x in json.load(open(base + "public.json"))]
-    assert verify_bls(vk, public, F.read_proof_json(base + "circom.proof"))
-    z = F.read_groth16_zkey(base + "circuit.zkey")
-    _, w = F.read_wtns(base + "witness.wtns")
+
+    def ref(rel):
+        return golden_fixture(tmp_path, rel)
+    base = "Groth16/bls12_381/poseidon/"
+    vk = F.read_vk_json(ref(base + "verification_key.json"))
+    public = [int(x) for x in json.load(open(ref(base + "public.json")))]
+    assert verify_bls(vk, public, F.read_proof_json(ref(base + "circom.proof")))
+    z = F.read_groth16_zkey(ref(base + "circuit.zkey"))
+    _, w = F.read_wtns(ref(base + "witness.wtns"))
     proof = OG.prove_plain(z, F.zkey_matrices(z), w, 1234567, 7654321)
     assert verify_bls(vk, public, proof)
-    base = REF + "/test_vectors/Plonk/bls12_381/poseidon/"
-    pvk = F.read_plonk_vk_json(base + "verification_key.json")
-    ppub = [int(x) for x in json.load(open(base + "public.json"))]
-    assert OP.verify(BLS12_381, pvk, F.read_plonk_proof_json(base + "circom.proof"), ppub, ppio)
+    base = "Plonk/bls12_381/poseidon/"
+    pvk = F.read_plonk_vk_json(ref(base + "verification_key.json"))
+    ppub = [int(x) for x in json.load(open(ref(base + "public.json")))]
+    assert OP.verify(BLS12_381, pvk, F.read_plonk_proof_json(ref(base + "circom.proof")), ppub, ppio)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF) or os.environ.get("CS_FULL_CPU_TESTS", "0") != "1",
-                    reason="needs the reference tree and takes ~20 s of big-int arithmetic: set CS_FULL_CPU_TESTS=1")
-def test_plonk_prover_bls12_381_poseidon_against_round1_kat_and_verifier():
+@pytest.mark.skipif(os.environ.get("CS_FULL_CPU_TESTS", "0") != "1",
+                    reason="takes ~20 s of big-int arithmetic: set CS_FULL_CPU_TESTS=1")
+def test_plonk_prover_bls12_381_poseidon_against_round1_kat_and_verifier(tmp_path):
     """The full oracle prover on the BLS12-381 poseidon fixture (domain 4096): its round-1 commitments are the
-    reference's known answers (co-plonk/src/round1.rs:397-417) and the whole proof passes Plonk::verify."""
+    reference's known answers (co-plonk/src/round1.rs:397-417), the proof is the stored one, and it passes
+    Plonk::verify under the fixture's verification key."""
     from oracle import plonk as OP
     from oracle.fields import BLS12_381
     from oracle.pairing_bls12_381 import pairing_product_is_one as ppio
-    base = REF + "/test_vectors/Plonk/bls12_381/poseidon/"
-    z = F.read_plonk_zkey(base + "circuit.zkey")
-    _, w = F.read_wtns(base + "witness.wtns")
+    z, w, gz = golden_plonk("poseidon", "bls12_381")
     pr = OP.prove(z, w)
     g = load_golden("plonk_round1_bls12_381_poseidon")
     assert [pr["a"], pr["b"], pr["c"]] == [gp1(P) for P in g["expected_commitments"]]
-    vk = F.read_plonk_vk_json(base + "verification_key.json")
-    assert OP.verify(BLS12_381, vk, pr, [int(x) for x in json.load(open(base + "public.json"))], ppio)
+    assert F.plonk_proof_to_json(pr, "bls12381") == gz["oracle_proof_json"]
+    base = "Plonk/bls12_381/poseidon/"
+    vk = F.read_plonk_vk_json(golden_fixture(tmp_path, base + "verification_key.json"))
+    assert OP.verify(BLS12_381, vk, pr, [int(x) for x in json.load(open(golden_fixture(tmp_path, base + "public.json")))], ppio)
 
 
 def test_chacha_published_known_answers():
